@@ -3,6 +3,10 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo (B200, sm_100a)
     python bench.py --impl reference --gpus N ...            # CPU baseline (oracle port)
+    python bench.py ... --dump-outputs DIR                   # + DIR/score.npy of the last timed step
+
+Inputs and weights come from fixed seeds, so two builds run with the same arguments can be
+compared output for output through --dump-outputs.
 
 Workload (BASELINE.json configs[1]): LanczosNet forward, config/qm8_lanczos_net.yaml,
 K=20 Ritz pairs, batch 1024 per GPU, synthetic QM8-shaped molecules (n_b in [3,26], N=26),
@@ -440,7 +444,14 @@ def main():
   ap.add_argument('--batch', type=int, default=BATCH)
   ap.add_argument('--no-cpu-baseline', action='store_true')
   ap.add_argument('--no-workloads', action='store_true')
+  ap.add_argument('--dump-outputs', metavar='DIR',
+                  help='after the timed steps, write the scores the last timed step returned '
+                       '(rank 0) as DIR/score.npy, float32 [batch, 16]')
   args = ap.parse_args()
+  if args.steps < 1:
+    ap.error('--steps must be at least 1')
+  if args.dump_outputs and args.impl != 'b200':
+    ap.error('--dump-outputs applies to --impl b200')
   args.warmup = max(args.warmup, 3) if args.impl == 'b200' else args.warmup
 
   if args.impl == 'reference':
@@ -515,6 +526,7 @@ def main():
     torch.cuda.synchronize(dev)
 
   def timed(fn, steps):
+    """CUDA-event ms of `steps` calls of fn (max over ranks) and the output of the last call."""
     del kept[:]
     barrier()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -528,8 +540,9 @@ def main():
     ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
     if world > 1:
       dist.all_reduce(ms, op=dist.ReduceOp.MAX)
+    last = kept[-1]
     del kept[:]
-    return float(ms.item())
+    return float(ms.item()), last
 
   with torch.no_grad():
     # correctness gate on this rank's first batch (small slice, CPU oracle as the checker)
@@ -561,11 +574,14 @@ def main():
     sampler = ClockSampler(local)
     sampler.start()
     l0 = ops.launch_count()
-    ms_total = timed(step_resident, args.steps)
+    ms_total, last_score = timed(step_resident, args.steps)
     launches = ops.launch_count() - l0
-    ms_e2e = timed(step_e2e, args.steps)
-    ms_e2e_dense = timed(step_e2e_dense, args.steps)
+    ms_e2e, _ = timed(step_e2e, args.steps)
+    ms_e2e_dense, _ = timed(step_e2e_dense, args.steps)
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+      os.makedirs(args.dump_outputs, exist_ok=True)
+      np.save(os.path.join(args.dump_outputs, 'score.npy'), last_score.float().cpu().numpy())
 
     # dominant kernel: the whole 7-layer spectral-conv stack + readout as ONE persistent tcgen05
     # kernel (K-depth 960 + 6 x 1920 per row), timed per launch with CUDA events on the
